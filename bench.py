@@ -14,8 +14,8 @@ entities = 2*n*E candidate triples scored.  metric = candidate triples scored pe
                  pinned HOST batch with `job._process_batch` — H2D of the triples, kernels, `.item()` D2H inside the
                  timed region (falls back to the C-ABI host entry point when LibKGE is not importable; `e2e.api` says)
   roofline     : dominant kernel, CUDA events on its launch stream, against MEASURED_PEAKS.json
-  cpu_baseline : the UNMODIFIED reference job (`model: complex`, job.device cpu, installed in baseline/_ref by
-                 scripts/install_ref.sh) processing the same batches on the host cores, bounded sample
+  cpu_baseline : the UNMODIFIED reference job (`model: complex`, job.device cpu, installed in oracle/_ref by
+                 oracle/install_ref.py) processing the same batches on the host cores, bounded sample
   configs      : (N=1) the other BASELINE.json configs — RotatE negative sampling, RESCAL KvsAll with CSR labels,
                  one Wikidata5M-shaped TransE shard — kernel ms, rate, roofline fraction, parity vs the live reference
   sharded      : (N>1) BASELINE config 5: TransE d=512, 600 k rows per GPU, entity-sharded across the N ranks with
@@ -35,6 +35,8 @@ import sys
 import tempfile
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -200,7 +202,7 @@ def _time_reference_job(steps, warmup, budget_s):
     per = sum(times) / len(times)
     return {"value": 2.0 * N_BATCH * E / per, "unit": UNIT, "cores": best_thr, "kind": "reference",
             "sample": f"{len(times)} x TrainingJob1vsAll._process_batch (forward only; n={N_BATCH}, E={E}, D={D}, BCE) "
-                      f"of the unmodified reference (baseline/_ref) on the host CPU, torch {torch.__version__}, "
+                      f"of the unmodified reference (oracle/_ref) on the host CPU, torch {torch.__version__}, "
                       f"{best_thr} threads (fastest of the probed thread counts on {cores_all} host cores)",
             "ms_per_step": per * 1e3, "avg_loss_last": loss}, len(times)
 
@@ -814,6 +816,7 @@ def run_ours(args):
     barrier()
     launches = engine.launch_count()
     engine.profile_enable(False)
+    outputs = {"loss": loss_dev.cpu().numpy()}      # the 0-d loss the last timed step returned
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -856,6 +859,9 @@ def run_ours(args):
         job_loss = step(i)                          # H2D + kernels + D2H (+ the job's own bookkeeping) inside
         e2e_t.append(time.perf_counter() - t0)
     barrier()
+    outputs["e2e_loss"] = np.float64(job_loss)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, "" if world == 1 else f"_rank{rank}")
     clocks = sampler.stop() if rank == 0 else None
     e2e_total = torch.tensor([sum(e2e_t)], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -940,6 +946,20 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, outputs, suffix=""):
+    """Writes each output as out_dir/<name><suffix>.npy (float32 / float64, at most 64 MB in all), so that two builds
+    run with the same arguments, and therefore the same seeded inputs, can be compared output for output."""
+    arrays = {name: np.asarray(a) for name, a in outputs.items()}
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"output {name} has dtype {a.dtype}; only float32 / float64 are dumped")
+    if sum(a.nbytes for a in arrays.values()) > 64 << 20:
+        raise ValueError("outputs exceed 64 MB; dump a seeded sample instead")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 _OUT_FD = None
 
 
@@ -969,7 +989,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configs (N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy: loss (the "
+                         "device-resident step) and e2e_loss (the host-batch step); with N > 1 each rank adds _rank<r>")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the device arm; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -2,14 +2,13 @@
 
 The plugin classes subclass the reference's own `KgeModel` / `TrainingJob*` classes, so `kge` must be
 importable.  In a LibKGE deployment it simply is (`pip install -e .`).  In this repository's test and bench
-environment the unmodified reference is installed by `scripts/install_ref.sh` into `baseline/_ref`
-(git-ignored; travels to the GPU box), and a handful of optional third-party modules that `kge` imports at
+environment build() installs the unmodified LibKGE into `oracle/_ref` (git-ignored; oracle/install_ref.py)
+when its source tree is present, and a handful of optional third-party modules that `kge` imports at
 module level but never touches on the training / evaluation path (`path`, `igraph`, `ConfigSpace`, `ax`,
 `hpbandster`, `sqlalchemy`, `torchviz`; SURVEY.md 8c) may be missing: those are replaced by empty stub
 modules — the reference code itself is not modified.
 
-Search order for the `kge` tree: `$KGE_REFERENCE_ROOT`, `<repo>/baseline/_ref`, an already importable `kge`,
-`/root/reference` (build container only).
+Search order for the `kge` tree: `$KGE_REFERENCE_ROOT`, `<repo>/oracle/_ref`, an already importable `kge`.
 """
 from __future__ import annotations
 
@@ -52,14 +51,10 @@ class _StubFinder(importlib.abc.MetaPathFinder, importlib.abc.Loader):
 
 def locate() -> str | None:
     """Directory that contains the `kge` package, or None if `kge` is importable as is / not found."""
-    cands = [os.environ.get("KGE_REFERENCE_ROOT"), os.path.join(_REPO, "baseline", "_ref")]
+    cands = [os.environ.get("KGE_REFERENCE_ROOT"), os.path.join(_REPO, "oracle", "_ref")]
     for c in cands:
         if c and os.path.isdir(os.path.join(c, "kge", "model")):
             return c
-    if "kge" in sys.modules or importlib.util.find_spec("kge") is not None:
-        return None
-    if os.path.isdir("/root/reference/kge/model"):
-        return "/root/reference"
     return None
 
 
@@ -78,7 +73,7 @@ def import_kge():
         if root is None and importlib.util.find_spec("kge") is None:
             raise ImportError(
                 "LibKGE (`kge`) is not importable: install it, set KGE_REFERENCE_ROOT, or run "
-                "scripts/install_ref.sh (installs the reference into baseline/_ref)")
+                "oracle/install_ref.py (installs it into oracle/_ref)")
         if root is not None and root not in sys.path:
             sys.path.insert(0, root)
         missing = []

@@ -1,8 +1,8 @@
-"""Import the live reference (uma-pi1/kge at /root/reference) inside the BUILD container.
+"""Import the live reference (uma-pi1/kge, installed into oracle/_ref by oracle/install_ref.py).
 
 TEST INFRASTRUCTURE.  Used only by tests/golden/gen_golden.py (to produce the committed
-golden vectors) and by CPU tests that are skipped when /root/reference is absent (it does
-not exist on the GPU box).  Nothing is copied from the reference: it is imported
+golden vectors) and by CPU tests that are skipped when the reference is not installed.
+Nothing is copied from the reference into the repository: it is imported
 read-only, with the five optional third-party modules it imports at module level but
 never touches on the scoring path (`path`, `igraph`, `ConfigSpace`, `ax`, `hpbandster`;
 SURVEY.md 8c) replaced by empty stub modules.
@@ -16,7 +16,8 @@ import sys
 import types
 import warnings
 
-REFERENCE_ROOT = os.environ.get("KGE_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("KGE_REFERENCE_ROOT",
+                                os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 class _StubModule(types.ModuleType):

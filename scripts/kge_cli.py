@@ -3,7 +3,7 @@
 
     python scripts/kge_cli.py start my-job.yaml --job.device cuda
 
-Locates the reference (installed LibKGE, $KGE_REFERENCE_ROOT or baseline/_ref — scripts/install_ref.sh), stubs the
+Locates the reference (installed LibKGE, $KGE_REFERENCE_ROOT or oracle/_ref — oracle/install_ref.py), stubs the
 optional third-party modules it imports at module level but does not use for training / evaluation, puts this
 repository on sys.path (so `modules: [..., kge_b200.plugin]` resolves) and hands over to kge.cli.main().  Nothing of
 LibKGE is modified."""

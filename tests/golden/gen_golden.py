@@ -1,12 +1,13 @@
-"""Generate golden vectors by running the LIVE reference (uma-pi1/kge) in the build container.
+"""Generate golden vectors by running the LIVE reference (uma-pi1/kge, installed into oracle/_ref by
+oracle/install_ref.py).
 
     python tests/golden/gen_golden.py          # writes tests/golden/*.npz
 
 The reference holds no golden vectors of its own for the scoring path (SURVEY.md 8c), so
 these files — outputs of the unmodified reference on seeded inputs — are what pins the
 oracle (tests/test_oracle_golden.py) and, through it and directly, the CUDA path
-(tests/test_gpu_*.py).  /root/reference does not exist on the GPU box; the committed .npz
-files travel instead.  Inputs are stored with the outputs so replay needs no RNG parity.
+(tests/test_gpu_*.py).  The tests need no reference installed: the committed .npz
+files stand in for it.  Inputs are stored with the outputs so replay needs no RNG parity.
 """
 from __future__ import annotations
 

@@ -1,4 +1,4 @@
-"""Helpers to run the UNMODIFIED reference jobs (LibKGE, installed by scripts/install_ref.sh into baseline/_ref)
+"""Helpers to run the UNMODIFIED reference jobs (LibKGE, installed by oracle/install_ref.py into oracle/_ref)
 on in-memory synthetic graphs — once as the reference itself (`model: <m>`, job.device cpu) and once through the
 kge_b200 plugin (`model: b200_<m>`, job.device cuda), with identical tables and identical batch order."""
 from __future__ import annotations

@@ -13,7 +13,7 @@ import torch.multiprocessing as mp
 
 from kge_b200 import hostenv
 
-pytestmark = pytest.mark.skipif(not hostenv.available(), reason="reference not installed (scripts/install_ref.sh)")
+pytestmark = pytest.mark.skipif(not hostenv.available(), reason="LibKGE not installed (oracle/install_ref.py)")
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 E, R, D = 53, 4, 16

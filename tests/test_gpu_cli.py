@@ -21,7 +21,7 @@ import yaml
 from kge_b200 import hostenv
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not hostenv.available(), reason="reference not installed (scripts/install_ref.sh)")]
+              pytest.mark.skipif(not hostenv.available(), reason="LibKGE not installed (oracle/install_ref.py)")]
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 E, R, SIZES = 280, 112, {"train": 4565, "valid": 109, "test": 152}

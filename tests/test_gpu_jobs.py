@@ -4,8 +4,8 @@ For every case the same job is run twice on the same in-memory graph with the sa
   (ref)  the reference itself:  model: <m>,       job.device: cpu
   (b200) through the plugin:    model: b200_<m>,  job.device: cuda   [+ optionally <type>.class_name: B200TrainingJob*]
 and the trace values are compared (avg_loss 1e-4 relative; ranking metrics: ranks agree for >= 99.5 % of the
-triples, which at these sizes means identical metrics).  Needs the reference installed in baseline/_ref
-(scripts/install_ref.sh — travels to the GPU box) and a B200.
+triples, which at these sizes means identical metrics).  Needs the reference installed in oracle/_ref
+(oracle/install_ref.py, run by build() when the LibKGE source tree is present) and a B200.
 """
 import pytest
 import torch
@@ -13,7 +13,7 @@ import torch
 from kge_b200 import hostenv
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not hostenv.available(), reason="reference not installed (scripts/install_ref.sh)")]
+              pytest.mark.skipif(not hostenv.available(), reason="LibKGE not installed (oracle/install_ref.py)")]
 
 import jobs_util as ju  # noqa: E402
 

@@ -56,7 +56,7 @@ def test_bench_reference_arm_runs_on_cpu():
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "triples/s" and line["value"] > 0
     from kge_b200 import hostenv
-    # the live reference's own job when it is installed (scripts/install_ref.sh), else the oracle's restatement
+    # the live reference's own job when it is installed (oracle/install_ref.py), else the oracle's restatement
     assert line["cpu_baseline"]["kind"] == ("reference" if hostenv.available() else "port")
     assert line["cpu_baseline"]["cores"] >= 1 and line["config"]["workload"].startswith("ComplEx d=512 1vsAll+BCE")
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["higher_is_better"] is True
@@ -212,3 +212,23 @@ def test_philox_reference_known_answers():
     assert philox4x32_10([0xffffffff] * 4, (0xffffffff, 0xffffffff)) == [0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd]
     assert philox4x32_10([0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344], (0xa4093822, 0x299f31d0)) == \
         [0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1]
+
+
+def test_reference_install_copies_modules_and_yaml_only(tmp_path, monkeypatch):
+    """oracle/install_ref.py installs LibKGE's modules and yaml data from a source tree, nothing else."""
+    from oracle import install_ref
+
+    src = tmp_path / "src"
+    for f in ("kge/__init__.py", "kge/model/__init__.py", "kge/model/complex.yaml", "kge/README.md", "setup.py"):
+        (src / f).parent.mkdir(parents=True, exist_ok=True)
+        (src / f).write_text(f)
+    monkeypatch.setattr(install_ref, "HERE", str(tmp_path))
+    monkeypatch.setattr(install_ref, "TARGET", str(tmp_path / "_ref"))
+    monkeypatch.setenv("KGE_REFERENCE_SRC", str(src))
+    assert install_ref.source_tree() == str(src) and not install_ref.installed()
+    install_ref.install(str(src))
+    got = sorted(str(p.relative_to(tmp_path / "_ref")) for p in (tmp_path / "_ref").rglob("*") if p.is_file())
+    assert got == ["kge/__init__.py", "kge/model/__init__.py", "kge/model/complex.yaml"]
+    assert install_ref.installed() and sorted(os.listdir(tmp_path)) == ["_ref", "src"]
+    with pytest.raises(RuntimeError):
+        install_ref.install(str(tmp_path / "_ref" / "kge"))      # no kge/model package below it

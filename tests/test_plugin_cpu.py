@@ -1,6 +1,6 @@
 """The LibKGE plugin loads through the reference's own plugin mechanism (config `modules:` +
 `<model>.yaml` class_name, kge/misc.py:13-42, kge_model.py:473-503).  Needs the live reference
-(/root/reference), which exists only in the build container; skipped elsewhere."""
+(installed into oracle/_ref by oracle/install_ref.py); skipped where it is not installed."""
 import pytest
 import torch
 

@@ -8,7 +8,7 @@ import torch
 
 from kge_b200 import hostenv
 
-pytestmark = pytest.mark.skipif(not hostenv.available(), reason="reference not installed (scripts/install_ref.sh)")
+pytestmark = pytest.mark.skipif(not hostenv.available(), reason="LibKGE not installed (oracle/install_ref.py)")
 
 import engine_stub  # noqa: E402
 import jobs_util as ju  # noqa: E402
